@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels through the C-ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one training step's worth of the hot path over one batch of 1024 synthetic quadruples:
 both directions (train.py:136-137) x both RGCN layers (Aggregator.py:136-137) over the batched history
@@ -93,7 +94,27 @@ def parse():
                          "as the line's value")
     ap.add_argument('--no-train', action='store_true', help='skip the training-step region of the default line')
     ap.add_argument('--dropout', type=float, default=0.0, help='dropout of the training-step region (reference default 0.5)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step of the aggregate, end-to-end and training '
+                         'regions returned as DIR/<name>.npy (float32/float64; the inputs are seeded, so two builds can be '
+                         'compared output for output)')
     return ap.parse_args()
+
+
+DUMP_MAX_ELEMS = 4 << 20      # per array (16 MB of float32): the at most four arrays of a dump stay within 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy.  One with more than DUMP_MAX_ELEMS elements is replaced by a fixed seeded
+    sample of its flattened elements: the same positions on every run of the same workload."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def algorithmic_bytes(N, E, R2):
@@ -274,7 +295,7 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------------
-def train_region(args, tkg, pool, global_emb, dev, world, torch, dist):
+def train_region(args, tkg, pool, global_emb, dev, world, torch, dist, outputs=None):
     """One reference training step per iteration (train.py:136-143) on this rank's shard of the global batch
     (1024 samples per rank, global batch 1024 x world): RENet.forward x2 directions -> backward through the CUDA
     backward kernels -> gradient all-reduce (NCCL, bucketed, launched from autograd hooks while backward still runs)
@@ -334,6 +355,8 @@ def train_region(args, tkg, pool, global_emb, dev, world, torch, dist):
         phases = tmax[2:].cpu().numpy()
         exposed_min = tmin[4].item()
     loss = float(torch.stack(losses).mean())
+    if outputs is not None:
+        outputs['train_loss'] = np.array([float(losses[-1])])
     tr.close()
     return {'value': msgs / (ms * 1e-3), 'unit': UNIT, 'ms_per_step': ms / args.steps, 'steps': args.steps, 'warmup': warm,
             'forward_ms': float(phases[0]), 'backward_ms': float(phases[1]), 'allreduce_exposed_ms': float(phases[2]),
@@ -412,11 +435,14 @@ def run_ours(args):
     msgs_per_step = [sum(2 * d['g'].E for d in e['dirs']) for e in pool]              # over the FULL E, as SURVEY 8(a) demands
     msgs_executed = [sum(d['g'].E + d['sub'].E for d in e['dirs']) for e in pool]     # edges the kernels actually walk
     pool_bytes = sum(sum(d['g'].E * 12 + d['g'].N * (8 + 1600) for d in e['dirs']) for e in pool)
+    outputs = {} if args.dump_outputs else None
     if args.mode == 'train':
         clocks = ClockSampler(local)
         clocks.start()
-        train = train_region(args, tkg, pool, model.global_emb, dev, world, torch, dist)
+        train = train_region(args, tkg, pool, model.global_emb, dev, world, torch, dist, outputs)
         clk = clocks.stop()
+        if rank == 0 and outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         if rank == 0:
             print(json.dumps({'metric': 'training_step_edge_messages_per_sec', 'value': train['value'], 'unit': UNIT, 'n_gpus': world,
                               'steps': args.steps, 'warmup': train['warmup'], 'ms_per_step': train['ms_per_step'],
@@ -487,6 +513,11 @@ def run_ours(args):
     launches = _lib.launch_count() - n0
     elapsed_ms = start.elapsed_time(end)
     clk = clocks.stop()
+    if outputs is not None:
+        # what the last timed step hands to the read-out: layer 2's output at every read-out row, in read-out order
+        # (Aggregator.py:140 keeps nothing else of it)
+        for d in pool[(args.warmup + args.steps - 1) % len(pool)]['dirs']:
+            outputs[('obj' if d['reverse'] else 'subj') + '_rgcn_readout'] = d['H2'][d['sub'].readout_c.long()].cpu().numpy()
     t = torch.tensor([elapsed_ms, float(total_msgs)], device=dev, dtype=torch.float64)
     if world > 1:
         tmax = t.clone(); dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -648,7 +679,7 @@ def run_ours(args):
             barrier()
             dt = time.perf_counter() - t0
             msgs = sum(2 * g.value() for g in graphs)
-            return h2d, d2h, msgs, dt
+            return h2d, d2h, msgs, dt, prev[1].clone()
 
         # loader threads per rank: 8 when the host has room; under a cgroup CPU quota leave a core per rank for the
         # consumer thread (a plan takes ~0.6 ms of one core, a step needs two: 2 threads keep up with a 1.3 ms step)
@@ -656,7 +687,7 @@ def run_ours(args):
         E2E_DEPTH = 4
         hoststore.reserve_pinned(4 * (E2E_DEPTH + 3))     # every staging buffer the loader can need, pinned up front
         E2E_WORKERS = max(2, min(8, _rank_cpu_budget() - int(os.environ.get('OMP_NUM_THREADS', '1')) - 1))
-        k_e2e = max(4, args.steps)
+        k_e2e = args.steps
         # one full rotation over the pool of batches: the loader, the pinned pool and the caching allocator (whose block
         # sizes depend on the batch) have reached steady state before the clock starts
         w_e2e = max(len(pool) + 1, args.warmup)
@@ -671,7 +702,9 @@ def run_ours(args):
                 buf = io.StringIO()
                 pstats.Stats(pr, stream=buf).sort_stats(key).print_stats(28)
                 sys.stderr.write(buf.getvalue())
-        h2d, d2h, msgs, dt = run_e2e(w_e2e, k_e2e, 0)
+        h2d, d2h, msgs, dt, last = run_e2e(w_e2e, k_e2e, 0)
+        if outputs is not None:
+            outputs['e2e_encode'] = last.numpy()      # [subject; object] x [s_h | s_q] of the last step, as RENet.encode returns them
         tt = torch.tensor([dt, float(msgs)], device=dev, dtype=torch.float64)
         if world > 1:
             a = tt.clone(); dist.all_reduce(a, op=dist.ReduceOp.MAX)
@@ -691,7 +724,7 @@ def run_ours(args):
     train = None
     if not args.no_train:
         try:
-            train = train_region(args, tkg, pool, model.global_emb, dev, world, torch, dist)
+            train = train_region(args, tkg, pool, model.global_emb, dev, world, torch, dist, outputs)
         except Exception as ex:          # the aggregate metric does not depend on it; a failure is reported, not hidden
             import traceback
             train = {'failed': '%s: %s' % (type(ex).__name__, ex), 'trace': traceback.format_exc()[-1500:]}
@@ -715,6 +748,8 @@ def run_ours(args):
                 'clocks': clk, 'e2e': e2e, 'gpu_launches': int(launches), 'roofline': roofline, 'cpu_baseline': cpu,
                 'gru_ms_one_direction': gru_ms, 'roofline_gemm': roofline_gemm, 'roofline_gru': roofline_gru, 'train': train}
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
 
@@ -724,6 +759,8 @@ if __name__ == '__main__':
     if a.timestamps is None:
         a.timestamps = WORKLOADS[a.workload][1]
     WORKLOAD = WORKLOADS[a.workload][2]
+    if a.dump_outputs and (a.workload == 'synth1m' or a.impl == 'reference'):
+        raise SystemExit('bench.py: --dump-outputs is implemented for --impl ours on the icews18 and gdelt workloads')
     if a.workload == 'synth1m' and a.impl != 'reference':
         from bench_synth import run_synth1m
         run_synth1m(a, WORKLOAD, METRIC, UNIT, ClockSampler, measured_peak_gbs)

@@ -150,6 +150,49 @@ def gen_layers(ns):
     print('layer_cases.npz: %d cases' % len(names))
 
 
+SAMPLE_ROWS = 32
+
+
+def random_layer_cases():
+    """Four random graphs for RE-Net's layer shape (d=200, nb=100, 32 relation types), rebuilt identically without the
+    reference: structure from one RandomState(0) stream, features and weights from seeded torch generators."""
+    rng = np.random.RandomState(0)
+    cases = []
+    for k in range(4):
+        N, E, R2 = int(rng.randint(1, 400)), int(rng.randint(1, 3000)), 32
+        src, dst = rng.randint(0, N, E), rng.randint(0, N, E)
+        ty = rng.randint(0, R2, E)
+        P = det_params({'weight': (R2, 4 * 100), 'loop_weight': (200, 200)}, 100 + k)
+        H = torch.randn(N, 200, generator=torch.Generator().manual_seed(200 + k))
+        cases.append(dict(N=N, src=src, dst=dst, ty=ty, H=H, W=P['weight'], Wloop=P['loop_weight']))
+    return cases
+
+
+def gen_random_layers(ns):
+    """Reference RGCNBlockLayer (relu, self-loop) on random_layer_cases(): its degree norm, and of each output the
+    max-abs, the float64 row and column sums and SAMPLE_ROWS seeded rows (all rows together would be 0.7 MB)."""
+    import torch.nn.functional as F
+    blob = {}
+    with ref_loader.cpu_patches():
+        for k, c in enumerate(random_layer_cases()):
+            layer = ns.RGCN.RGCNBlockLayer(200, 200, 32, 100, activation=F.relu, self_loop=True)
+            with torch.no_grad():
+                layer.weight.copy_(c['W'])
+                layer.loop_weight.copy_(c['Wloop'])
+            g = ns.dgl.DGLGraph(); g.add_nodes(c['N']); g.add_edges(c['src'], c['dst'])
+            g.ndata['norm'] = ns.utils.comp_deg_norm(g).view(-1, 1)
+            g.edata['type_s'] = torch.as_tensor(c['ty']); g.edata['type_o'] = torch.as_tensor(c['ty'])
+            g.ndata['h'] = c['H'].clone()
+            layer(g, False)
+            out = g.ndata['h'].detach().numpy()
+            rows = np.sort(np.random.RandomState(k).choice(c['N'], min(c['N'], SAMPLE_ROWS), replace=False))
+            blob.update({'%d/norm' % k: g.ndata['norm'].view(-1).numpy(), '%d/rows' % k: rows, '%d/out_rows' % k: out[rows],
+                         '%d/absmax' % k: np.abs(out).max(), '%d/rowsum' % k: out.astype(np.float64).sum(1),
+                         '%d/colsum' % k: out.astype(np.float64).sum(0)})
+    np.savez_compressed(os.path.join(OUT, 'reference_random_layers.npz'), **blob)
+    print('reference_random_layers.npz: %d cases' % len(random_layer_cases()))
+
+
 RENET_SHAPES = lambda num_e, h, R, nb: {  # noqa: E731
     'rel_embeds': (2 * R, h), 'ent_embeds': (num_e, h),
     'encoder.weight_ih_l0': (3 * h, 4 * h), 'encoder.weight_hh_l0': (3 * h, h),
@@ -536,3 +579,4 @@ if __name__ == '__main__':
     gen_aggregator_predict(ns)
     gen_global_tiny(ns)
     gen_renet_eval_global(ns)
+    gen_random_layers(ns)

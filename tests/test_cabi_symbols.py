@@ -50,7 +50,9 @@ def test_argument_validation_needs_no_gpu(so_path):
 
 
 def test_sass_is_sm100a(so_path):
-    out = subprocess.run(['cuobjdump', '-lelf', so_path], capture_output=True, text=True).stdout
+    from renet_b200 import build
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), 'cuobjdump')     # the toolkit that built the library
+    out = subprocess.run([cuobjdump, '-lelf', so_path], capture_output=True, text=True).stdout
     assert 'sm_100a' in out, out
 
 
