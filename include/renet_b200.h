@@ -41,7 +41,9 @@ const char* renet_last_error(void);
 int64_t renet_launch_count(void);
 
 /* Dense-GEMM engine used for the self-loop and GRU projections: 0 = FFMA (fp32 CUDA cores),
- * 1 = tcgen05 3xTF32 (tensor cores, fp32-accurate split).  Both are this library's own kernels.
+ * 1 = tcgen05 3xTF32 (tensor cores, fp32-accurate split; the self-loop shape N = K = 200 runs a persistent kernel),
+ * 2 = tcgen05 3xTF32 with the general packed kernel for every shape (the self-loop kernel before the persistent one;
+ * same results, kept for A/B timing).  All are this library's own kernels.
  * Process-wide; the initial value comes from the RENET_GEMM environment variable (ffma|umma).
  * renet_set_gemm_engine returns the previous engine. */
 int renet_set_gemm_engine(int engine);

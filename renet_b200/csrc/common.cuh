@@ -82,7 +82,7 @@ constexpr int64_t kStreamMaxNodes = 98304;    // 79 MB of fp32 features: beyond 
 bool gather_use_stream(int64_t E, int64_t N);
 void set_stream_debug_buffer(long long* p);   // debug: per-warp time stamps of the stream kernel (rgcn_fwd.cu)          // the stream kernel (rgcn_stream.cuh) serves this edge count
 
-// tcgen05 GEMM engine building blocks (umma_gemm.cu); gemm_mode() == 1 selects the engine
+// tcgen05 GEMM engine building blocks (umma_gemm.cu); gemm_mode() != 0 selects the engine (2: no persistent self-loop kernel)
 int gemm_mode();
 int64_t umma_packed_bytes(int N, int K);
 // packed-weight cache (umma_gemm.cu): persistent device buffer for this key, or nullptr when caching is off; *hit says

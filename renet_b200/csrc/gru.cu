@@ -289,7 +289,7 @@ int launch_gru_fwd(const float* H2, const int32_t* readout, const int32_t* row_g
   const bool dropout = p_drop > 0.f || dense;
   GruWs w = carve(ws_base, S, Q, T, h, kMaxLenWs, dropout);
   {
-    const bool splittable = gemm_mode() == 1 && h % 4 == 0 && (3 * h) % 200 == 0 && (reinterpret_cast<uintptr_t>(ws_base) & 127) == 0 &&
+    const bool splittable = gemm_mode() != 0 && h % 4 == 0 && (3 * h) % 200 == 0 && (reinterpret_cast<uintptr_t>(ws_base) & 127) == 0 &&
                             !dropout;
     if (!splittable) {
       if (phase == 1) return RENET_OK;
@@ -316,7 +316,7 @@ int launch_gru_fwd(const float* H2, const int32_t* readout, const int32_t* row_g
   // Tensor-core engine: weights go straight into the UMMA operand image (hi/lo planes, K-major, 128-byte swizzle),
   // ONCE per call -- the recurrent weights are re-used by every time step -- and every GEMM is one launch; the two
   // encoders' recurrent GEMMs are batched into a single launch per step.
-  const bool use_umma = gemm_mode() == 1 && h % 4 == 0 && (3 * h) % 200 == 0 &&
+  const bool use_umma = gemm_mode() != 0 && h % 4 == 0 && (3 * h) % 200 == 0 &&
                         (reinterpret_cast<uintptr_t>(ws_base) & 127) == 0;
   if (use_umma) {
     const int t3 = 3 * h / 200;   // column tiles per encoder
@@ -641,7 +641,7 @@ int launch_gru_bwd(const float* H2, const int32_t* readout, const int32_t* row_g
   const int64_t hs_stride = Q * 2 * h;
   const int64_t gh_stride = Q * 6 * h;
   // tensor-core engine: W_hh of both encoders packed ONCE as the B operand of dHprev += dGH @ W_hh (B[k][n] = w_hh[k*h + n])
-  const bool use_umma = gemm_mode() == 1 && umma_shape_ok(h, 3 * h) && (reinterpret_cast<uintptr_t>(b.P_hhT) & 127) == 0;
+  const bool use_umma = gemm_mode() != 0 && umma_shape_ok(h, 3 * h) && (reinterpret_cast<uintptr_t>(b.P_hhT) & 127) == 0;
   if (use_umma && last > 1) {
     if ((rc = umma_pack_b(w_hh4, h, 1, h, 3 * h, b.P_hhT, 0, stream))) return rc;
     if ((rc = umma_pack_b(w_hh3, h, 1, h, 3 * h, reinterpret_cast<uint8_t*>(b.P_hhT) + b.p_hht_bytes, 0, stream))) return rc;

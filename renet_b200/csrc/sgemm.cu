@@ -239,7 +239,9 @@ int umma_gemm_nn_try(const float* A, const int32_t* a_index, int64_t lda, const 
                      int64_t ldc, const float* bias, int64_t M, int32_t N, int32_t K, bool accumulate,
                      cudaStream_t stream);
 
-// RENET_GEMM=ffma|umma selects the dense-GEMM engine (both are this library's own sm_100a kernels).
+// RENET_GEMM=ffma|umma selects the dense-GEMM engine (all are this library's own sm_100a kernels): 0 = FFMA, 1 = tensor
+// cores (the self-loop shape on its persistent kernel); renet_set_gemm_engine(2) = tensor cores with the packed kernel for
+// every shape (the previous self-loop kernel, kept for A/B comparisons).
 static int g_gemm_mode = -1;
 int gemm_mode() {
   if (g_gemm_mode < 0) {
@@ -250,7 +252,7 @@ int gemm_mode() {
 }
 int set_gemm_mode(int m) {
   const int prev = gemm_mode();
-  g_gemm_mode = m ? 1 : 0;
+  g_gemm_mode = m == 2 ? 2 : (m ? 1 : 0);
   return prev;
 }
 
@@ -258,7 +260,7 @@ int sgemm_nn(const float* A, const int32_t* a_index, int64_t lda, const float* B
              int64_t ldc, const float* bias, int64_t M, int32_t N, int32_t K, bool accumulate,
              cudaStream_t stream) {
   if (M <= 0 || N <= 0) return RENET_OK;
-  if (gemm_mode() == 1) {   // tcgen05 3xTF32 path (umma_gemm.cu); returns 0 when the shape is not supported
+  if (gemm_mode() != 0) {   // tcgen05 3xTF32 path (umma_gemm.cu); returns 0 when the shape is not supported
     const int r = umma_gemm_nn_try(A, a_index, lda, B, ldb, C, ldc, bias, M, N, K, accumulate, stream);
     if (r != 0) return r < 0 ? r : RENET_OK;
   }

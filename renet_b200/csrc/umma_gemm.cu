@@ -506,6 +506,274 @@ umma_gemm_packed_kernel(const float* __restrict__ A, const int32_t* __restrict__
   }
 }
 
+// ======================================================================================================
+// v3: the self-loop product C[M, 200] = A[idx[m]] @ W_loop (N = 200, one packed column tile; no bias, no accumulate)
+//
+// The packed kernel runs stage-A / MMA rounds separated by CTA-wide barriers followed by a serial epilogue, and gives
+// every CTA 256 rows: a layer-2 shape (S ~ 8.5k rows) occupies 34 of 148 SMs.  This kernel is persistent and
+// warp-specialised:
+//   * grid = min(units, SMs); CTA b owns units b, b + grid, b + 2 grid, ... (at most ceil(units / grid) each);
+//   * a unit is 128 rows x all 208 columns; when the row tiles fill at most half of the SMs, a unit is 128 rows x one
+//     column half instead: N = 112 (columns 0..111) or N = 96 (112..207).  Both are legal M = 128 MMA widths and both
+//     start on a 1024-byte swizzle atom of the packed image (row 112 = 14 KB), so TMA fetches just that half's rows;
+//   * roles, all hand-offs on mbarriers (no CTA-wide barrier in the main loop):
+//       warps 0-7    gather the A rows through the index, split hi/lo, store them swizzled into a 3-stage ring;
+//       warp 8       (one lane) streams the packed B chunks with cp.async.bulk into a 2-stage ring;
+//       warp 9       (one lane) issues the MMAs and commits; it also owns the TMEM allocation;
+//       warps 10-13  drain the accumulators (warp w reads TMEM lanes 32 (w % 4) ..);
+//   * two TMEM accumulators (columns [0, 256) and [256, 512)): unit i's epilogue overlaps unit i+1's MMAs;
+//   * the last K chunk issues only the k-steps that carry data (1 of 4 for K = 200).  The products keep the packed
+//     kernel's order (per k-step hi.hi, lo.hi, hi.lo; k ascending): the skipped k-steps only added zeros;
+//   * epilogue: tcgen05.ld of 32 rows x 32 columns -> a per-warp padded shared tile -> 128-byte row segments to C.
+// Shared memory (bytes): A ring 3 x 32768 + B ring 2 x 53248 + epilogue 4 x 4608 + barriers 128 + alignment 1024
+// = 224384 (219 KB of the 227 KB a block may have).
+constexpr int SL_PROD_WARPS = 8;
+constexpr int SL_PROD = SL_PROD_WARPS * 32;
+constexpr int SL_TMA_WARP = 8;
+constexpr int SL_MMA_WARP = 9;
+constexpr int SL_EPI_WARP0 = 10;
+constexpr int SL_THREADS = (SL_EPI_WARP0 + 4) * 32;      // 448
+constexpr int SL_A_STAGES = 3;
+constexpr int SL_B_STAGES = 2;
+constexpr int SL_A_STAGE = 2 * P_A_BYTES;                 // hi + lo planes of 128 rows x 32 k
+constexpr int SL_EPI_LD = 36;                             // floats per staged row: 32 + 4 keeps 16-byte accesses conflict-free
+constexpr int SL_EPI_WARP_BYTES = 32 * SL_EPI_LD * 4;     // 4608
+constexpr int SL_OFF_B = SL_A_STAGES * SL_A_STAGE;
+constexpr int SL_OFF_EPI = SL_OFF_B + SL_B_STAGES * P_B_CHUNK;
+constexpr int SL_OFF_BAR = SL_OFF_EPI + 4 * SL_EPI_WARP_BYTES;
+constexpr int SL_SMEM = SL_OFF_BAR + 128 + 1024;
+constexpr int SL_HALF0_N = 112;                           // width of the first column half; the second is UNP - 112 = 96
+static_assert(SL_SMEM <= 227 * 1024, "self-loop kernel: shared memory budget");
+static_assert((SL_HALF0_N * 128) % 1024 == 0, "column half must start on a swizzle atom");
+// mbarrier slots (8 bytes each) after SL_OFF_BAR
+constexpr int SL_BAR_A_FULL = 0, SL_BAR_A_EMPTY = 3, SL_BAR_B_FULL = 6, SL_BAR_B_EMPTY = 8, SL_BAR_T_FULL = 10,
+              SL_BAR_T_EMPTY = 12, SL_NUM_BARS = 14;
+
+struct SlUnit {
+  int64_t row0;   // first row of the 128-row tile
+  int col0;       // first accumulator column within the 208-column tile
+  int n;          // MMA width: 208, 112 or 96
+};
+__device__ __forceinline__ SlUnit sl_unit(int u, int split) {
+  SlUnit s;
+  if (split) {
+    s.row0 = (int64_t)(u >> 1) * UM;
+    s.col0 = (u & 1) ? SL_HALF0_N : 0;
+    s.n = (u & 1) ? UNP - SL_HALF0_N : SL_HALF0_N;
+  } else {
+    s.row0 = (int64_t)u * UM;
+    s.col0 = 0;
+    s.n = UNP;
+  }
+  return s;
+}
+
+template <bool INDEXED>
+__global__ void __launch_bounds__(SL_THREADS, 1)
+umma_selfloop_kernel(const float* __restrict__ A, const int32_t* __restrict__ a_index, int64_t lda,
+                     const uint8_t* __restrict__ Bp, float* __restrict__ C, int64_t ldc, int64_t M, int K, int n_chunks,
+                     int n_units, int split) {
+  extern __shared__ uint8_t smem_raw[];
+  const uint32_t raw = smem_u32(smem_raw);
+  uint8_t* smem = smem_raw + ((1024 - (raw & 1023)) & 1023);     // swizzle atoms need 1024-byte alignment
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const uint32_t smem_base = smem_u32(smem);
+  const uint32_t bar0 = smem_base + SL_OFF_BAR;
+  auto bar = [&](int i) { return bar0 + 8 * i; };
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + SL_OFF_BAR + 8 * SL_NUM_BARS);
+
+  if (tid == 0) {
+    for (int s = 0; s < SL_A_STAGES; ++s) {
+      mbar_init(bar(SL_BAR_A_FULL + s), SL_PROD);
+      mbar_init(bar(SL_BAR_A_EMPTY + s), 1);
+    }
+    for (int s = 0; s < SL_B_STAGES; ++s) {
+      mbar_init(bar(SL_BAR_B_FULL + s), 1);
+      mbar_init(bar(SL_BAR_B_EMPTY + s), 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(bar(SL_BAR_T_FULL + a), 1);
+      mbar_init(bar(SL_BAR_T_EMPTY + a), 128);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == SL_MMA_WARP) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  const uint32_t tmem_base = *tmem_slot;
+
+  const int n_local = (n_units - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // >= 1: grid <= n_units
+  const int total = n_local * n_chunks;                                                  // (unit, K chunk) items
+  const int last_ks = (K - (n_chunks - 1) * P_BK + 7) / 8;                              // k-steps of the last chunk
+
+  if (warp < SL_PROD_WARPS) {
+    // ---- A producers: 128 rows x 8 sixteen-byte chunks per K chunk = 4 tasks per thread; 8 consecutive lanes read one
+    // 128-byte row segment (coalesced) and write 8 distinct swizzled chunks (conflict-free).  The global loads of item
+    // it+1 are issued before item it is stored, and before waiting for its stage to be free.
+    const int j = tid & 7;
+    uint32_t a_off[4];
+#pragma unroll
+    for (int t = 0; t < 4; ++t) a_off[t] = sw128_offset((tid >> 3) + 32 * t, j);
+    const float* rows[4];
+    float4 vnext[4];
+    auto set_rows = [&](int lu) {
+      const SlUnit un = sl_unit((int)blockIdx.x + lu * (int)gridDim.x, split);
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        const int64_t gr = un.row0 + (tid >> 3) + 32 * t;
+        rows[t] = nullptr;
+        if (gr < M) rows[t] = A + (INDEXED ? (int64_t)__ldg(a_index + gr) : gr) * lda;
+      }
+    };
+    auto load = [&](int c) {
+      const int k = c * P_BK + 4 * j;
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        vnext[t] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (rows[t] != nullptr && k < K) vnext[t] = ldg_f4(rows[t] + k);
+      }
+    };
+    set_rows(0);
+    load(0);
+    for (int it = 0; it < total; ++it) {
+      const int s = it % SL_A_STAGES, round = it / SL_A_STAGES;
+      float4 v[4];
+#pragma unroll
+      for (int t = 0; t < 4; ++t) v[t] = vnext[t];
+      if (it + 1 < total) {
+        const int lu = (it + 1) / n_chunks, c = it + 1 - lu * n_chunks;
+        if (c == 0) set_rows(lu);
+        load(c);
+      }
+      if (round > 0) mbar_wait(bar(SL_BAR_A_EMPTY + s), (round - 1) & 1);   // the MMAs of item it-3 have read the stage
+      uint8_t* sA_hi = smem + s * SL_A_STAGE;
+      uint8_t* sA_lo = sA_hi + P_A_BYTES;
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        float4 hi, lo;
+        split4(v[t], hi, lo);
+        *reinterpret_cast<float4*>(sA_hi + a_off[t]) = hi;
+        *reinterpret_cast<float4*>(sA_lo + a_off[t]) = lo;
+      }
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");         // generic-proxy writes -> async proxy (MMA)
+      asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(SL_BAR_A_FULL + s)) : "memory");
+    }
+  } else if (warp == SL_TMA_WARP) {
+    if (lane == 0) {
+      // ---- B: one (unit, chunk) item = the chunk's packed block, or the rows of the unit's column half of it --------
+      for (int it = 0; it < total; ++it) {
+        const int s = it % SL_B_STAGES, round = it / SL_B_STAGES;
+        const int lu = it / n_chunks, c = it - lu * n_chunks;
+        const SlUnit un = sl_unit((int)blockIdx.x + lu * (int)gridDim.x, split);
+        if (round > 0) mbar_wait(bar(SL_BAR_B_EMPTY + s), (round - 1) & 1);
+        const uint32_t full = bar(SL_BAR_B_FULL + s);
+        const uint32_t dst = smem_base + SL_OFF_B + s * P_B_CHUNK;
+        const uint8_t* src = Bp + (size_t)c * P_B_CHUNK + un.col0 * 128;
+        const uint32_t plane = (uint32_t)un.n * 128;
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(2 * plane) : "memory");
+        if (un.n == UNP) {      // full width: the hi and lo planes are contiguous
+          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
+                       "l"(src), "r"((uint32_t)P_B_CHUNK), "r"(full)
+                       : "memory");
+        } else {
+#pragma unroll
+          for (int p = 0; p < 2; ++p)
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                             dst + p * P_B_BYTES),
+                         "l"(src + p * P_B_BYTES), "r"(plane), "r"(full)
+                         : "memory");
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp == SL_MMA_WARP) {
+    if (lane == 0) {
+      int it = 0;
+      for (int lu = 0; lu < n_local; ++lu) {
+        const int acc = lu & 1;
+        const SlUnit un = sl_unit((int)blockIdx.x + lu * (int)gridDim.x, split);
+        const uint32_t idesc = make_idesc_n(un.n);
+        if (lu >= 2) mbar_wait(bar(SL_BAR_T_EMPTY + acc), ((lu >> 1) - 1) & 1);   // epilogue of unit lu-2 has drained it
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        const uint32_t d = tmem_base + acc * 256;
+        for (int c = 0; c < n_chunks; ++c, ++it) {
+          const int sa = it % SL_A_STAGES, sb = it % SL_B_STAGES;
+          mbar_wait(bar(SL_BAR_A_FULL + sa), (it / SL_A_STAGES) & 1);
+          mbar_wait(bar(SL_BAR_B_FULL + sb), (it / SL_B_STAGES) & 1);
+          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          const uint32_t a_hi = smem_base + sa * SL_A_STAGE, a_lo = a_hi + P_A_BYTES;
+          const uint32_t b_hi = smem_base + SL_OFF_B + sb * P_B_CHUNK, b_lo = b_hi + P_B_BYTES;
+          const int nks = (c == n_chunks - 1) ? last_ks : P_BK / 8;
+          for (int ks = 0; ks < nks; ++ks) {
+            const uint32_t ko = ks * 32;                       // 8 fp32 = 32 bytes along the swizzled row
+            const uint64_t dAh = make_desc_sw128(a_hi + ko), dAl = make_desc_sw128(a_lo + ko);
+            const uint64_t dBh = make_desc_sw128(b_hi + ko), dBl = make_desc_sw128(b_lo + ko);
+            umma_tf32(d, dAh, dBh, idesc, (c | ks) != 0);
+            umma_tf32(d, dAl, dBh, idesc, 1);
+            umma_tf32(d, dAh, dBl, idesc, 1);
+          }
+          umma_commit(bar(SL_BAR_A_EMPTY + sa));               // both stages may be overwritten once these MMAs are done
+          umma_commit(bar(SL_BAR_B_EMPTY + sb));
+        }
+        umma_commit(bar(SL_BAR_T_FULL + acc));                 // accumulator complete
+      }
+    }
+    __syncwarp();
+  } else {
+    // ---- epilogue: TMEM -> registers (thread = row, 32 columns) -> padded shared tile -> 8 lanes per 128-byte row segment
+    const int q = warp & 3;
+    float* stg = reinterpret_cast<float*>(smem + SL_OFF_EPI + (warp - SL_EPI_WARP0) * SL_EPI_WARP_BYTES);
+    for (int lu = 0; lu < n_local; ++lu) {
+      const int acc = lu & 1;
+      const SlUnit un = sl_unit((int)blockIdx.x + lu * (int)gridDim.x, split);
+      const int col_end = min(UN, un.col0 + un.n);
+      const int nblk = (un.n + 31) / 32;
+      mbar_wait(bar(SL_BAR_T_FULL + acc), (lu >> 1) & 1);
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      const uint32_t taddr = tmem_base + acc * 256 + ((uint32_t)(q * 32) << 16);
+#pragma unroll 1
+      for (int blk = 0; blk < nblk; ++blk) {
+        uint32_t v[32];
+        asm volatile(
+            "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
+            "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
+              "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
+              "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
+              "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
+            : "r"(taddr + (uint32_t)(blk * 32)));
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        if (blk == nblk - 1) {     // every column of this accumulator is in registers: the MMAs may reuse it
+          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+          asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(SL_BAR_T_EMPTY + acc)) : "memory");
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+          *reinterpret_cast<uint4*>(stg + lane * SL_EPI_LD + 4 * i) = make_uint4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
+        __syncwarp();
+#pragma unroll
+        for (int p = 0; p < 8; ++p) {
+          const int r = 4 * p + (lane >> 3), c4 = lane & 7;
+          const int64_t gr = un.row0 + q * 32 + r;
+          const int gc = un.col0 + blk * 32 + 4 * c4;
+          if (gr < M && gc < col_end) st_f4(C + gr * ldc + gc, *reinterpret_cast<const float4*>(stg + r * SL_EPI_LD + 4 * c4));
+        }
+        __syncwarp();
+      }
+    }
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == SL_MMA_WARP) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
+  }
+}
+
 }  // namespace
 
 // Returns 1 if the shape was taken by the tensor-core path (launch enqueued), 0 if the caller should
@@ -621,6 +889,39 @@ int umma_gemm_prepacked(const float* A, const int32_t* a_index, int64_t lda, con
   return r < 0 ? r : RENET_OK;
 }
 
+// C[M, 200] = A[(a_index)] @ Bpacked with the persistent self-loop kernel (v3 above).
+static int umma_selfloop(const float* A, const int32_t* a_index, int64_t lda, const void* Bp, float* C, int64_t ldc,
+                         int64_t M, int K, cudaStream_t stream) {
+  static bool attr = false;
+  if (!attr) {
+    RENET_CHECK_CUDA(cudaFuncSetAttribute(umma_selfloop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM));
+    RENET_CHECK_CUDA(cudaFuncSetAttribute(umma_selfloop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SL_SMEM));
+    attr = true;
+  }
+  static int sm_count[64] = {0};
+  int dev = 0;
+  RENET_CHECK_CUDA(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= 64) dev = 0;
+  if (sm_count[dev] == 0) RENET_CHECK_CUDA(cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
+  const int sms = sm_count[dev];
+  const int64_t tiles = (M + UM - 1) / UM;
+  // Column halves double the units (and read every A row twice); they pay off only while the whole-width units leave
+  // at least half of the SMs idle.
+  const int split = 2 * tiles <= sms ? 1 : 0;
+  const int64_t units = split ? 2 * tiles : tiles;
+  RENET_CHECK_ARG(units < (int64_t)1 << 30, "umma_selfloop: too many rows");
+  const int grid = (int)(units < sms ? units : sms);
+  const int n_chunks = (K + P_BK - 1) / P_BK;
+  if (a_index)
+    umma_selfloop_kernel<true><<<grid, SL_THREADS, SL_SMEM, stream>>>(A, a_index, lda, (const uint8_t*)Bp, C, ldc, M, K,
+                                                                     n_chunks, (int)units, split);
+  else
+    umma_selfloop_kernel<false><<<grid, SL_THREADS, SL_SMEM, stream>>>(A, a_index, lda, (const uint8_t*)Bp, C, ldc, M, K,
+                                                                      n_chunks, (int)units, split);
+  RENET_CHECK_LAUNCH("umma_selfloop_kernel");
+  return RENET_OK;
+}
+
 int umma_gemm_nn_try(const float* A, const int32_t* a_index, int64_t lda, const float* B, int64_t ldb, float* C,
                      int64_t ldc, const float* bias, int64_t M, int32_t N, int32_t K, bool accumulate,
                      cudaStream_t stream) {
@@ -636,7 +937,11 @@ int umma_gemm_nn_try(const float* A, const int32_t* a_index, int64_t lda, const 
     void* Bp = cached ? cached : g_scratch;
     int rc = hit ? 0 : umma_pack_b(B, ldb, 1, N, K, Bp, 0, stream);
     if (rc) return rc;
-    rc = umma_gemm_prepacked(A, a_index, lda, Bp, C, ldc, bias, M, N, K, accumulate, 1, 0, 0, 0, stream);
+    // the self-loop shape (H @ W_loop, RGCN.py:35) takes the persistent kernel unless engine 2 asks for the packed one
+    if (gemm_mode() == 1 && N == UN && K == UN && bias == nullptr && !accumulate)
+      rc = umma_selfloop(A, a_index, lda, Bp, C, ldc, M, K, stream);
+    else
+      rc = umma_gemm_prepacked(A, a_index, lda, Bp, C, ldc, bias, M, N, K, accumulate, 1, 0, 0, 0, stream);
     return rc ? rc : 1;
   }
   const bool ok = (K % UKC == 0) && K >= UKC && (N % 8 == 0) && (lda % 4 == 0) && (ldb % 4 == 0) && (ldc % 4 == 0) &&
